@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the hot path's headline benchmark (BASELINE.json: "GFLOP/s at N=K=M=16384 fp32").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 One step = one MatrixMultiplicationKernel invocation C = A * B (operand preparation + GEMM, or the
 configured semiring) over one batch of synthetic matrices through the C-ABI of libmm_b200.so.
@@ -17,6 +17,8 @@ Printed JSON line (rank 0): see the contract in the task statement; in addition
   e2e           the same metric through ONE host-pointer call for the whole problem, H2D + D2H inside: mm_gemm_host()
                 at N = 1, mm_multi_gemm_host() over all N GPUs (issued by rank 0) at N > 1
 `--impl reference` times only the reference CPU path (oracle/_ref; the oracle port if absent).
+`--dump-outputs DIR` writes the C of the last timed step to DIR (dump_rows) so that two builds can be compared
+output for output: the inputs are drawn from fixed seeds, identical on every run with the same arguments.
 """
 import argparse
 import ctypes
@@ -301,6 +303,25 @@ def cpu_baseline_line(dtype_name, mp_name, rd_name, unit, k, m, a_rows_of, b):
             "seconds": secs, "host_cpus": os.cpu_count(), "sample": cpu_sample_text(rows, k, cols, threads)}
 
 
+DUMP_BYTES = 64 * 10 ** 6   # --dump-outputs writes at most this much in all
+
+
+def dump_rows(directory, name, c, budget):
+    """Write the device matrix `c` as DIR/<name>.npy in float32 (float64 for double): every row when they fit `budget`
+    bytes, otherwise a sample of rows drawn with a fixed seed (the same rows on every run of the same shape).  The
+    indices of the written rows go beside it as DIR/<name>_rows.npy (float64, exact)."""
+    import numpy as np
+    import torch
+    wide = torch.float64 if c.dtype == torch.float64 else torch.float32
+    n, m = c.shape
+    row_bytes = m * torch.empty((), dtype=wide).element_size()
+    keep = min(n, (budget - 4096) // (row_bytes + 8))   # 4096: room for the two .npy headers
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name + ".npy"), c[torch.from_numpy(rows).to(c.device)].to(wide).cpu().numpy())
+    np.save(os.path.join(directory, name + "_rows.npy"), rows.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -315,7 +336,13 @@ def main():
     ap.add_argument("--emulate-ranks", type=int, default=0,
                     help="experiments only: time ONE rank's row-block of an R-GPU split on this GPU (N/R rows); "
                          "the printed value is that block's own rate, not a multi-GPU figure")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write C of the last timed step as DIR/c.npy (a fixed row sample when larger than 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -506,6 +533,8 @@ def main():
         rows = torch.tensor([0, n_local // 2, n_local - 1], device=dev)
         extra["check"] = "3 rows of C vs fp64 torch.matmul on device: max rel err %.2e" % check_rows(c_blk[rows], a_blk[rows],
                                                                                                  "device-timed", b_use)
+    if args.dump_outputs:   # every rank writes its own block of C
+        dump_rows(args.dump_outputs, "c" if world == 1 else "c_rank%d" % rank, c_blk, DUMP_BYTES // world)
 
     out = None
     if rank == 0:
